@@ -6,9 +6,12 @@ the same descriptors to the CUDA kernel and to this library and compare bytes.
 
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB = os.path.join(HERE, "_build", "liboracle_copy_rects.so")
@@ -16,25 +19,40 @@ LIB = os.path.join(HERE, "_build", "liboracle_copy_rects.so")
 _lib = None
 
 
+def _writable_dir(path: str) -> bool:
+    try:
+        os.makedirs(path, exist_ok=True)
+    except OSError:
+        return False
+    return os.access(path, os.W_OK)
+
+
 def build(force: bool = False) -> str:
+    """Compile the oracle into oracle/_build when it is missing or older than its sources; returns the
+    library's path.  A checkout that cannot be written (bench.py may run from a read-only tree) gets
+    the rebuild in a temporary directory, removed at exit."""
     src = os.path.join(HERE, "copy_rects_ref.c")
     hdr = os.path.join(os.path.dirname(HERE), "include", "tstore_b200.h")
     stale = (not os.path.exists(LIB)) or os.path.getmtime(LIB) < max(os.path.getmtime(src), os.path.getmtime(hdr))
-    if force or stale:
-        os.makedirs(os.path.dirname(LIB), exist_ok=True)
-        cmd = ["gcc", "-O2", "-fPIC", "-shared", "-pthread", "-std=gnu11", "-I", os.path.dirname(hdr), "-o", LIB + ".tmp", src]
-        proc = subprocess.run(cmd, capture_output=True, text=True)
-        if proc.returncode != 0:
-            raise RuntimeError(f"oracle build failed:\n{proc.stdout}\n{proc.stderr}")
-        os.replace(LIB + ".tmp", LIB)
-    return LIB
+    if not (force or stale):
+        return LIB
+    out = LIB
+    if not _writable_dir(os.path.dirname(LIB)):
+        tmp_dir = tempfile.mkdtemp(prefix="tsb_oracle_")
+        atexit.register(shutil.rmtree, tmp_dir, True)
+        out = os.path.join(tmp_dir, os.path.basename(LIB))
+    cmd = ["gcc", "-O2", "-fPIC", "-shared", "-pthread", "-std=gnu11", "-I", os.path.dirname(hdr), "-o", out + ".tmp", src]
+    proc = subprocess.run(cmd, capture_output=True, text=True)
+    if proc.returncode != 0:
+        raise RuntimeError(f"oracle build failed:\n{proc.stdout}\n{proc.stderr}")
+    os.replace(out + ".tmp", out)
+    return out
 
 
 def lib() -> C.CDLL:
     global _lib
     if _lib is None:
-        build()
-        h = C.CDLL(LIB)
+        h = C.CDLL(build())
         h.oracle_copy_rects.restype = C.c_int
         h.oracle_copy_rects.argtypes = [C.c_void_p, C.c_uint64, C.c_int, C.c_int]
         h.oracle_copy_rects_pinned.restype = C.c_int

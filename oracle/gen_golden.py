@@ -14,7 +14,12 @@ Fixtures (all produced by reference code, not by the oracle or the product):
   store_reshard.json  LocalClient + Controller + InMemoryStore + SharedMemoryTransportBuffer:
                       put shards / reshard-get for the mesh pairs of tests/test_resharding_basic.py,
                       tests/test_resharding_ext.py and tests/test_tensor_slice.py (sha256 of results)
+  reference_dropin.json  DirectWeightSyncDest._build_plan op lists for handles that carry our
+                      NvlinkBuffer, plus the field names of RDMAWeightHandle / TensorSlice and the
+                      methods the reference calls on a handle's rdma_buffer
   cast_vectors.npz    torch CPU .to() bit patterns for the dtype pairs the cast kernel implements
+
+``python oracle/gen_golden.py NAME ...`` regenerates only the named fixtures.
 """
 
 from __future__ import annotations
@@ -455,6 +460,84 @@ def gen_store_reshard():
 
 
 # ------------------------------------------------------------------------------------------------
+def gen_reference_dropin():
+    """The reference's _build_plan fed handles that carry our NvlinkBuffer (descriptor only, as a
+    destination process sees them after unpickling); tests/test_reference_dropin.py builds our plan
+    from the same handles and compares it op for op."""
+    import dataclasses
+    import inspect
+    import re
+
+    import torchstore.direct_weight_sync as ref
+    from torchstore.transport.types import TensorSlice
+
+    import workloads
+    from torchstore_b200 import direct_weight_sync as ours
+    from torchstore_b200.planner import HbmDescriptor
+
+    def fake_buffer(shape, device):
+        stride = [int(np.prod(shape[i + 1:])) for i in range(len(shape))]
+        desc = HbmDescriptor(region=bytes(120), shape=tuple(shape), stride=tuple(stride), dtype=torch.float32, device=device)
+        return ours.NvlinkBuffer(descriptor=desc)
+
+    def make_slice(shape, n, r, placement):
+        off, shp = workloads.shard_box(shape, n, r, placement) if placement[0] == "S" else ((0,) * len(shape), tuple(shape))
+        return TensorSlice(offsets=tuple(off), coordinates=(r,), global_shape=tuple(shape), local_shape=tuple(shp), mesh_shape=(n,))
+
+    # (global shape, n source ranks, source placement, n dest ranks, dest placement)
+    cases = [
+        ((512, 512), 2, ("S", 0), 2, ("S", 0)),   # exact
+        ((512, 512), 4, ("S", 0), 2, ("S", 1)),   # reshard
+        ((96, 40), 4, ("S", 0), 3, ("S", 1)),     # uneven
+        ((64,), 4, ("R",), 2, ("R",)),            # replicated dedup
+        ((128, 64), 8, ("S", 0), 1, ("R",)),      # replicated reader (config 3)
+    ]
+    out = {"cases": []}
+    for shape, n_src, sp, n_dst, dp in cases:
+        per_dest = {}
+        for drank in range(n_dst):
+            ds = make_slice(shape, n_dst, drank, dp)
+            if 0 in ds.local_shape:
+                continue
+            handles, rank_of = [], {}
+            for r in range(n_src):
+                ss = make_slice(shape, n_src, r, sp)
+                if 0 in ss.local_shape:
+                    continue
+                buf = fake_buffer(ss.local_shape, r)
+                rank_of[id(buf)] = r
+                handles.append(ref.RDMAWeightHandle(rdma_buffer=buf, tensor_slice=ss, source_rank=r))
+            dest = torch.zeros(ds.local_shape, dtype=torch.float32)
+            # a plain destination tensor stands for "the whole tensor"; hand the reference the shard's
+            # slice the way Request.from_dtensor would
+            saved = ref._request_to_slice
+            ref._request_to_slice = lambda req, param, _s=ds: _s
+            try:
+                plan = ref.DirectWeightSyncDest()._build_plan({"w": handles}, {"w": dest})
+            finally:
+                ref._request_to_slice = saved
+            ops = []
+            for op in plan:
+                exact = op.dest_tensor is None
+                ops.append({
+                    "source_rank": rank_of[id(op.rdma_buffer)],
+                    "exact": exact,
+                    "src_index": None if exact else [[s.start, s.stop] for s in op.src_slices],
+                    "dest_index": None if exact else [[s.start, s.stop] for s in op.dest_slices],
+                    "recv_shape": None if exact else list(op.recv_buffer.shape),
+                    # exact: the read lands in the caller's tensor; partial: the overlap is copied into it
+                    "writes_into_dest": (op.dest_byte_view.data_ptr() == dest.data_ptr()) if exact else (op.dest_tensor is dest),
+                })
+            per_dest[str(drank)] = ops
+        out["cases"].append({"global_shape": list(shape), "n_src": n_src, "src_placement": list(sp), "n_dst": n_dst,
+                             "dst_placement": list(dp), "ops_by_dest_rank": per_dest})
+    out["handle_fields"] = [f.name for f in dataclasses.fields(ref.RDMAWeightHandle)]
+    out["tensor_slice_fields"] = [f.name for f in dataclasses.fields(TensorSlice)]
+    out["buffer_calls"] = sorted(set(re.findall(r"\.rdma_buffer\.(\w+)\(", inspect.getsource(ref))))
+    return out
+
+
+# ------------------------------------------------------------------------------------------------
 def gen_cast_vectors():
     rng = np.random.default_rng(7)
     edge32 = np.array([
@@ -493,14 +576,23 @@ def main():
     ref_harness.import_reference()
     os.makedirs(GOLDEN, exist_ok=True)
     meta = {"reference_commit": "ed2ddb67", "torch": torch.__version__, "generator": "oracle/gen_golden.py"}
-    for name, fn in (("slice_math", gen_slice_math), ("direct_plan", gen_direct_plan), ("store_reshard", gen_store_reshard)):
+    fixtures = {"slice_math": gen_slice_math, "direct_plan": gen_direct_plan, "store_reshard": gen_store_reshard,
+                "reference_dropin": gen_reference_dropin}
+    wanted = sys.argv[1:] or [*fixtures, "cast_vectors"]
+    unknown = set(wanted) - set(fixtures) - {"cast_vectors"}
+    if unknown:
+        raise SystemExit(f"unknown fixtures {sorted(unknown)}; choose from {[*fixtures, 'cast_vectors']}")
+    for name, fn in fixtures.items():
+        if name not in wanted:
+            continue
         data = fn()
         data["_meta"] = meta
         with open(os.path.join(GOLDEN, name + ".json"), "w") as f:
             json.dump(data, f, separators=(",", ":"))
         print(name, os.path.getsize(os.path.join(GOLDEN, name + ".json")), "bytes")
-    np.savez_compressed(os.path.join(GOLDEN, "cast_vectors.npz"), **gen_cast_vectors())
-    print("cast_vectors", os.path.getsize(os.path.join(GOLDEN, "cast_vectors.npz")), "bytes")
+    if "cast_vectors" in wanted:
+        np.savez_compressed(os.path.join(GOLDEN, "cast_vectors.npz"), **gen_cast_vectors())
+        print("cast_vectors", os.path.getsize(os.path.join(GOLDEN, "cast_vectors.npz")), "bytes")
 
 
 if __name__ == "__main__":

@@ -17,6 +17,7 @@ def test_reference_arm_prints_contract_line():
     assert len(lines) == 1
     d = json.loads(lines[0])
     assert d["impl"] == "reference" and d["unit"] == "GB/s" and d["value"] > 0 and d["higher_is_better"] is True
+    assert d["steps"] == 2 and d["warmup"] == 1
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
     assert d["config"]["state_dict_bytes"] == 16060522496

@@ -1,39 +1,31 @@
-"""Drop-in proof, build container only (the reference does not travel to the GPU box): our
-``NvlinkBuffer`` handles go through the reference's UNMODIFIED ``DirectWeightSyncDest._build_plan``
-(metadata only -- /root/reference/torchstore/direct_weight_sync.py:221-317) and the op list it
-builds must equal the one our own ``_build_plan`` builds from the same handles: same length, same
-order, same exact/partial classification, same source/destination slices, same buffer per op.
+"""Drop-in proof: our ``NvlinkBuffer`` handles go through the reference's UNMODIFIED
+``DirectWeightSyncDest._build_plan`` (metadata only -- torchstore/direct_weight_sync.py:221-317) and
+the op list it builds must equal the one our own ``_build_plan`` builds from the same handles: same
+length, same order, same exact/partial classification, same source/destination slices, same buffer
+per op.  The reference's op lists were recorded by oracle/gen_golden.py into
+tests/golden/reference_dropin.json.
 
-Also checks the other half of the duck-type contract (direct_weight_sync.py:46-58): an
-``RDMAWeightHandle`` carrying an ``NvlinkBuffer`` survives the pickle round trip every store put
-performs, and exposes the coroutine methods the reference calls (read_into / write_from / drop).
+Also checks the other half of the duck-type contract (direct_weight_sync.py:46-58): a handle with the
+reference's fields carrying an ``NvlinkBuffer`` survives the pickle round trip every store put
+performs, and the buffer exposes the coroutine methods the reference calls (read_into / write_from / drop).
 """
 
+import dataclasses
 import inspect
+import json
+import os
 import pickle
 
 import pytest
 import torch
 
-from oracle import ref_harness
+import workloads
 from torchstore_b200 import direct_weight_sync as ours
 from torchstore_b200.planner import HbmDescriptor
 from torchstore_b200.transport.types import TensorSlice as OurSlice
 
-pytestmark = pytest.mark.skipif(not ref_harness.reference_available(), reason="reference tree not present (GPU box)")
-
-import workloads  # noqa: E402
-
-
-@pytest.fixture(autouse=True)
-def _restore_sys_path():
-    """import_reference() puts /root/reference first on sys.path; it has its own ``tests`` package,
-    which must not shadow ours in processes spawned by later tests."""
-    import sys
-
-    saved = list(sys.path)
-    yield
-    sys.path[:] = saved
+with open(os.path.join(os.path.dirname(__file__), "golden", "reference_dropin.json")) as _f:
+    GOLDEN = json.load(_f)
 
 
 def _fake_buffer(shape, dtype, device):
@@ -48,12 +40,10 @@ def _fake_buffer(shape, dtype, device):
 
 
 def _cases():
-    # (global shape, n source ranks, source placement, n dest ranks, dest placement)
-    yield (512, 512), 2, ("S", 0), 2, ("S", 0)      # exact
-    yield (512, 512), 4, ("S", 0), 2, ("S", 1)      # reshard
-    yield (96, 40), 4, ("S", 0), 3, ("S", 1)        # uneven
-    yield (64,), 4, ("R",), 2, ("R",)               # replicated dedup
-    yield (128, 64), 8, ("S", 0), 1, ("R",)         # replicated reader (config 3)
+    # (global shape, n source ranks, source placement, n dest ranks, dest placement, recorded reference ops)
+    for c in GOLDEN["cases"]:
+        yield (tuple(c["global_shape"]), c["n_src"], tuple(c["src_placement"]), c["n_dst"], tuple(c["dst_placement"]),
+               c["ops_by_dest_rank"])
 
 
 def _slice(cls, shape, n, r, placement):
@@ -61,60 +51,58 @@ def _slice(cls, shape, n, r, placement):
     return cls(offsets=tuple(off), coordinates=(r,), global_shape=tuple(shape), local_shape=tuple(shp), mesh_shape=(n,))
 
 
+def _slices(index):
+    return tuple(slice(a, b) for a, b in index)
+
+
 @pytest.mark.parametrize("case", list(_cases()), ids=lambda c: f"{c[0]}-{c[1]}{c[2]}->{c[3]}{c[4]}")
-def test_reference_build_plan_accepts_nvlink_buffers_and_matches_ours(case, monkeypatch):
-    shape, n_src, sp, n_dst, dp = case
-    ref_harness.import_reference()
-    import torchstore.direct_weight_sync as ref
-    from torchstore.transport.types import TensorSlice as RefSlice
+def test_reference_build_plan_accepts_nvlink_buffers_and_matches_ours(case):
+    shape, n_src, sp, n_dst, dp, ref_ops_by_rank = case
 
     for drank in range(n_dst):
-        bufs = []
-        ref_handles, our_handles = [], []
+        buf_of_rank, our_handles = {}, []
         for r in range(n_src):
-            rs = _slice(RefSlice, shape, n_src, r, sp)
+            rs = _slice(OurSlice, shape, n_src, r, sp)
             if 0 in rs.local_shape:
                 continue
             buf = _fake_buffer(rs.local_shape, torch.float32, r)
-            bufs.append(buf)
-            ref_handles.append(ref.RDMAWeightHandle(rdma_buffer=buf, tensor_slice=rs, source_rank=r))
-            our_handles.append(ours.RDMAWeightHandle(rdma_buffer=buf, tensor_slice=_slice(OurSlice, shape, n_src, r, sp), source_rank=r))
-        ds_ref = _slice(RefSlice, shape, n_dst, drank, dp)
+            buf_of_rank[r] = buf
+            our_handles.append(ours.RDMAWeightHandle(rdma_buffer=buf, tensor_slice=rs, source_rank=r))
         ds_our = _slice(OurSlice, shape, n_dst, drank, dp)
-        if 0 in ds_ref.local_shape:
+        if 0 in ds_our.local_shape:
             continue
-        dest = torch.zeros(ds_ref.local_shape, dtype=torch.float32)
-        # the reference derives the destination slice from a DTensor; a plain tensor stands for "the
-        # whole tensor", so hand it the shard's slice the way Request.from_dtensor would
-        monkeypatch.setattr(ref, "_request_to_slice", lambda req, param, _s=ds_ref: _s)
-        ref_ops = ref.DirectWeightSyncDest()._build_plan({"w": ref_handles}, {"w": dest})
+        ref_ops = ref_ops_by_rank[str(drank)]
+        dest = torch.zeros(ds_our.local_shape, dtype=torch.float32)
         our_ops = ours.DirectWeightSyncDest()._build_plan({"w": our_handles}, {"w": dest}, {"w": ds_our})
         assert len(ref_ops) == len(our_ops) > 0
         for a, b in zip(ref_ops, our_ops):
-            assert a.rdma_buffer is b.rdma_buffer  # same source, same order
-            ref_exact = a.dest_tensor is None
+            assert buf_of_rank[a["source_rank"]] is b.rdma_buffer  # same source, same order
+            ref_exact = a["exact"]
             assert ref_exact == (b.dest_tensor is None)
+            assert a["writes_into_dest"]  # the reference fills the caller's tensor, not a copy of it
             if not ref_exact:
-                assert tuple(a.src_slices) == tuple(b.src_slices)
-                assert tuple(a.dest_slices) == tuple(b.dest_slices)
-                assert a.dest_tensor is dest and b.dest_tensor is dest
+                assert _slices(a["src_index"]) == tuple(b.src_slices)
+                assert _slices(a["dest_index"]) == tuple(b.dest_slices)
+                assert b.dest_tensor is dest
                 # the reference stages the WHOLE source shard; we describe just the overlap rectangle
-                assert tuple(a.recv_buffer.shape) == tuple(a.rdma_buffer.shape)
+                assert tuple(a["recv_shape"]) == tuple(buf_of_rank[a["source_rank"]].shape)
             else:
-                assert a.dest_byte_view.data_ptr() == b.dest_byte_view.data_ptr() == dest.data_ptr()
+                assert b.dest_byte_view.data_ptr() == dest.data_ptr()
 
 
 def test_handle_pickles_and_duck_types_like_an_rdma_buffer():
-    ref_harness.import_reference()
-    import torchstore.direct_weight_sync as ref
-    from torchstore.transport.types import TensorSlice as RefSlice
+    # our handle and slice carry exactly the reference's fields, so either side can build the other's
+    assert [f.name for f in dataclasses.fields(ours.RDMAWeightHandle)] == GOLDEN["handle_fields"]
+    assert [f.name for f in dataclasses.fields(OurSlice)] == GOLDEN["tensor_slice_fields"]
 
     buf = _fake_buffer((16, 8), torch.bfloat16, 3)
-    h = ref.RDMAWeightHandle(rdma_buffer=buf, tensor_slice=_slice(RefSlice, (32, 8), 2, 1, ("S", 0)), source_rank=1)
+    h = ours.RDMAWeightHandle(**dict(zip(GOLDEN["handle_fields"], (buf, _slice(OurSlice, (32, 8), 2, 1, ("S", 0)), 1))))
     h2 = pickle.loads(pickle.dumps(h))
     assert h2.rdma_buffer.descriptor == buf.descriptor and h2.tensor_slice == h.tensor_slice and h2.source_rank == 1
     assert h2.rdma_buffer.nbytes == 16 * 8 * 2 and h2.rdma_buffer.dtype == torch.bfloat16
-    for name in ("read_into", "write_from", "drop"):  # call sites direct_weight_sync.py:143,174,339
+    methods = ("read_into", "write_from", "drop")  # call sites direct_weight_sync.py:143,174,339
+    assert set(GOLDEN["buffer_calls"]) <= set(methods)
+    for name in methods:
         assert inspect.iscoroutinefunction(getattr(h2.rdma_buffer, name))
     # CPU tensors are refused loudly (no host data plane behind this handle)
     import asyncio
